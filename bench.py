@@ -4,6 +4,7 @@
   python bench.py --gpus N --steps K --warmup W            # the CUDA path (default workload)
   python bench.py --impl reference ...                     # the reference's own CPU path
   python bench.py --workload waymo_mv | waymo_10sweep      # BASELINE.json configs[3] / [4]
+  python bench.py ... --dump-outputs DIR                   # + last timed step's outputs, .npy
 
 Workloads (one "step" = one pass of the hot path over one synthetic input):
   kitti          BASELINE.json configs[1]: one KITTI-shape pair, 370x1224 padded to 384x1248,
@@ -46,6 +47,14 @@ V = D * HO * WO
 FLOPS_PER_FRAME = 521856.0 * V                       # SURVEY.md 8(d)
 IO_BYTES_PER_FRAME = 2 * 32 * H * W * 4 + 5.25e6 + 33 * V * 4
 KITTI_WORKLOAD = 'dfm_r34_1x8_kitti-3d-3class D=112 384x1248 batch=1'
+# what one kitti step hands its caller: DfMBackbone's (cost, stereo, mono), DepthHead's 3 outputs
+KITTI_OUTPUTS = ('cost', 'stereo_feat', 'mono_feat', 'depth_volumes', 'depth_volumes_softmax',
+                 'depth_preds')
+# --dump-outputs: an output with more elements than this is stored as a fixed, seeded sample;
+# six outputs of at most 8 MiB each stay within DUMP_MAX_BYTES
+DUMP_MAX_ELEMS = 1 << 21
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SEED = 0
 # dram__bytes_read.sum + dram__bytes_write.sum of one launch of the dominant kernel, from the
 # committed `ncu --set full` capture (profiles/): kitti: conv_tc 32->32 full resolution
 NCU_TRAFFIC = {'kitti': (973.0e6, 'profiles/r02_ncu_conv_tc_dominant_final.csv '
@@ -67,6 +76,31 @@ def peaks():
         return dict(bf16=j.get('bf16_tflops_sustained', j.get('bf16_tflops')),
                     hbm=j.get('hbm_gbs'), src='measured')
     return dict(bf16=1400.0, hbm=6650.0, src='fallback')  # B200_PROFILING.md
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each named output as ``<out_dir>/<name>.npy`` (float32 or float64), so that two
+    builds run with the same arguments can be compared output for output.  An output with at
+    most DUMP_MAX_ELEMS elements is written whole, in its own shape; a larger one as the 1-D
+    array of its elements at DUMP_MAX_ELEMS flat indices drawn (with replacement, then sorted)
+    from a CPU generator seeded with DUMP_SEED, which depend only on the output's size."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMS:
+            g = torch.Generator().manual_seed(DUMP_SEED)
+            idx = torch.randint(t.numel(), (DUMP_MAX_ELEMS,), generator=g).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        a = t.cpu().numpy()
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float32)
+        total += a.nbytes
+        if total > DUMP_MAX_BYTES:
+            raise RuntimeError(f'--dump-outputs: more than {DUMP_MAX_BYTES} bytes at {name}')
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 class ClockSampler:
@@ -183,8 +217,11 @@ def run_reference(args):
     ts = []
     for _ in range(args.steps):
         t0 = time.perf_counter()
-        step()
+        last = step()
         ts.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        name = 'depth_preds' if args.workload == 'kitti' else 'volume_feat'
+        dump_outputs(args.dump_outputs, {name: last})
     per_step = sum(ts) / len(ts)
     fps = 1.0 / per_step
     name = KITTI_WORKLOAD if args.workload == 'kitti' else WAYMO[args.workload]['name']
@@ -255,7 +292,8 @@ def _setup_dist():
 
 def _timed_loop(step, args, world, rank, local, capi):
     """W warm-up steps, then exactly K timed steps between barrier + synchronize on both
-    sides, CUDA events on the launching stream, clocks sampled during the timed region."""
+    sides, CUDA events on the launching stream, clocks sampled during the timed region.
+    Also returns what the last timed step returned."""
     import torch
     import torch.distributed as dist
 
@@ -277,8 +315,9 @@ def _timed_loop(step, args, world, rank, local, capi):
             sampler.start()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for i in range(args.steps):
+        for i in range(args.steps - 1):
             step(i)
+        last = step(args.steps - 1)
         e1.record()
         barrier()
         clocks = sampler.stop() if rank == 0 else None
@@ -288,7 +327,7 @@ def _timed_loop(step, args, world, rank, local, capi):
         l1, tc1 = capi.launch_counters()
         capi.sync_check()
     from depth_from_motion_b200.sharding import reduce_step_time
-    return reduce_step_time(ms, 'cuda'), prof, clocks, l1 - l0, tc1 - tc0, barrier
+    return reduce_step_time(ms, 'cuda'), prof, clocks, l1 - l0, tc1 - tc0, barrier, last
 
 
 def _kernel_table(prof, steps):
@@ -329,11 +368,14 @@ def run_kitti(args):
     def step(i):
         cur, prev, metas, _, _ = pairs[i % 2]
         cost, stereo, mono = model(cur, prev, metas)
-        return head(cost)
+        return (cost, stereo, mono) + tuple(head(cost))
 
-    ms_total, prof, clocks, launches, tc_launches, barrier = _timed_loop(
+    ms_total, prof, clocks, launches, tc_launches, barrier, last = _timed_loop(
         step, args, world, rank, local, capi)
     fps = world * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(KITTI_OUTPUTS, last)))
+    del last
 
     # ---- e2e: DfM.simple_test's hot-path segment through the host-buffer C-ABI call -------
     # pinned host (cur, prev, sem) in -> voxel features + depth_preds out (what the BEV stage
@@ -540,9 +582,12 @@ def run_waymo(args):
         feats, meta, _ = samples[i % 2]
         return host.feature_transformation(feats[None], [meta], nv, t)[0]
 
-    ms_total, prof, clocks, launches, tc_launches, barrier = _timed_loop(
+    ms_total, prof, clocks, launches, tc_launches, barrier, last = _timed_loop(
         step, args, world, rank, local, capi)
     sps = world * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(volume_feat=last))
+    del last
 
     # ---- e2e: pinned host features in, pinned host BEV out --------------------------------
     # every step copies its sample H2D (166 / 83 MB) and its BEV map D2H (67.6 MB) inside the timed
@@ -675,7 +720,11 @@ def main():
     ap.add_argument('--workload', default='kitti', choices=['kitti'] + sorted(WAYMO))
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-gpu-eager', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the outputs of the last timed step to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.warmup = max(args.warmup, 3)
     if args.impl == 'reference':
         run_reference(args)

@@ -10,6 +10,7 @@ reference's own DfMBackbone / DepthHead / DfMNeck / OutdoorImVoxelNeck /
 FrustumToVoxel / point_sample code returns on CPU in fp32.
 """
 import copy
+import json
 import os
 import sys
 
@@ -162,9 +163,143 @@ def frustum_case(ns):
           float((out != 0).float().mean()))
 
 
+def state_dict_layout_case(ns):
+    """Key order and shapes of the reference modules' state_dicts (the on-disk checkpoint
+    contract the mirrors in depth_from_motion_b200/modules.py must keep)."""
+    from tests.util import STATE_DICT_MODULES
+    layout = {name: [[k, list(v.shape)] for k, v in make(ns).state_dict().items()]
+              for name, make in STATE_DICT_MODULES.items()}
+    with open(os.path.join(HERE, 'state_dict_layout.json'), 'w') as f:
+        json.dump(layout, f, indent=0)
+        f.write('\n')
+    print('state_dict_layout', {k: len(v) for k, v in layout.items()})
+
+
+def config_blocks_case(ref_root):
+    """The hot-path blocks of the `model` dict of each shipped configs/dfm/*.py, as parsed."""
+    from depth_from_motion_b200 import registry
+    from tests.util import CONFIG_MODEL_BLOCKS, DFM_CONFIGS
+    out = {}
+    for name in DFM_CONFIGS:
+        model = registry.Config.fromfile(os.path.join(ref_root, 'configs/dfm', name)).model
+        out[name] = {k: model[k] for k in CONFIG_MODEL_BLOCKS[model['type']]}
+    with open(os.path.join(HERE, 'config_model_blocks.json'), 'w') as f:
+        json.dump(out, f, indent=1)
+        f.write('\n')
+    print('config_model_blocks', {k: sorted(v) for k, v in out.items()})
+
+
+def voxel_sample_case(ns):
+    """The reference voxel_sample (point_fusion.py:324-410, executed verbatim) on the inputs
+    of tests/util.py:voxel_sample_args."""
+    import torch.nn.functional as F
+    from oracle.ref_loader import reference_function
+    from tests.util import voxel_sample_args
+    ref = reference_function('mmdet3d/models/fusion_layers/point_fusion.py', 'voxel_sample',
+                             dict(torch=torch, F=F, points_img2cam=ns.points_img2cam))
+    out = {}
+    for flip, aligned in ((False, True), (True, True), (False, False)):
+        out[f'flip{int(flip)}_aligned{int(aligned)}'] = \
+            ref(*voxel_sample_args(flip), aligned=aligned).numpy()
+    np.savez_compressed(os.path.join(HERE, 'voxel_sample.npz'), **out)
+    print('voxel_sample', {k: v.shape for k, v in out.items()})
+
+
+def bev_stage_small_case(ns):
+    """Reference BEVHourglass + LIGAAnchor3DHead.forward_single on tests/util.py:BEV_SMALL_CASE
+    (a 12 x 16 BEV grid)."""
+    from tests.util import BEV_SMALL_CASE
+    c = syn.make_bev_case(**BEV_SMALL_CASE)
+    gn = dict(type='GN', num_groups=32, requires_grad=True)
+    bev = ns.BEVHourglass(160, 64, norm_cfg=gn).eval()
+    head = ns.LIGAAnchor3DHead(3, 64, 64, 6, norm_cfg=gn).eval()
+    bev.load_state_dict(c['bev'], strict=True)
+    head.load_state_dict(c['head'], strict=True)
+    with torch.no_grad():
+        _, feat = bev(c['volume'].reshape(1, 160, 12, 16))
+        cls, box, dirc = head.forward_single(feat)
+    np.savez_compressed(os.path.join(HERE, 'bev_stage_small.npz'), cls_score=cls.numpy(),
+                        bbox_pred=box.numpy(), dir_cls_preds=dirc.numpy())
+    print('bev_stage_small', tuple(cls.shape), tuple(box.shape), tuple(dirc.shape))
+
+
+def spp_lastconv_case(ns):
+    """Reference SPPUNetNeck.lastconv (spp_unet_neck.py:60-75, :110): its parameters as the
+    reference initialises them, and its output on tests/util.py:spp_lastconv_input."""
+    from tests.util import spp_lastconv_input
+    gn = dict(type='GN', num_groups=32, requires_grad=True)
+    m = ns.SPPUNetNeck(in_channels=[3, 64, 128, 128, 128], start_level=2, sem_channels=[128, 32],
+                       stereo_channels=[32, 32], with_upconv=True, cat_img_feature=True,
+                       norm_cfg=gn).eval()
+    p = {k: v.numpy() for k, v in m.state_dict().items() if k.startswith('lastconv')}
+    with torch.no_grad():
+        y = m.lastconv(spp_lastconv_input())
+    np.savez_compressed(os.path.join(HERE, 'spp_unet_lastconv.npz'), y=y.numpy(), **p)
+    print('spp_unet_lastconv', sorted(p), tuple(y.shape))
+
+
+def pipeline_meta_case(ref_root):
+    """The reference VideoPipeline (loading.py) on the geometry of its demo KITTI sample, and
+    RandomCrop3D._crop_data (transforms_3d.py), both executed verbatim."""
+    import pickle
+    from oracle.ref_loader import reference_class
+    with open(os.path.join(ref_root, 'demo/data/kitti/kitti_000008_infos.pkl'), 'rb') as f:
+        info = pickle.load(f)[0]
+    img_info = dict(filename='x.png', cam2global=info['image']['cam2global'],
+                    sweeps=[dict(data_path=s['data_path'], cam2global=s['cam2global'])
+                            for s in info['image']['sweeps']])
+
+    class Compose:   # the image transforms are out of scope: identity
+        def __init__(self, t):
+            pass
+
+        def __call__(self, r):
+            r['img'] = 0
+            return r
+
+    VP = reference_class('mmdet3d/datasets/pipelines/loading.py', 'VideoPipeline',
+                         dict(np=np, copy=copy, Compose=Compose))
+    out = dict(cam2global=np.asarray(img_info['cam2global'], np.float64),
+               sweep_cam2global=np.stack([s['cam2global'] for s in img_info['sweeps']]),
+               sweep_paths=np.array([s['data_path'] for s in img_info['sweeps']]))
+    for nref, rand in ((1, False), (3, False), (2, True)):
+        np.random.seed(7)
+        ref = VP([], num_ref_imgs=nref, random=rand)(dict(img_info=copy.deepcopy(img_info)))
+        out[f'cur2prevs_n{nref}_random{int(rand)}'] = np.asarray(ref['cur2prevs'])
+
+    class RandomCrop:   # mmdet base: only what _crop_data touches
+        def __init__(self, **kw):
+            self.bbox_clip_border = kw.get('bbox_clip_border', True)
+            self.bbox2label, self.bbox2mask = {}, {}
+
+    RC = reference_class('mmdet3d/datasets/pipelines/transforms_3d.py', 'RandomCrop3D',
+                         dict(np=np, RandomCrop=RandomCrop))
+    rc = RC(crop_size=(320, 1280), rel_offset_h=(0.3, 1.0))
+    img = np.zeros((375, 1242, 3), dtype=np.uint8)
+    np.random.seed(3)
+    ref = rc._crop_data(dict(img=img, cam2img=syn.KITTI_P2.copy()), (320, 1280), True)
+    out.update(crop_offset=np.asarray(ref['crop_offset']),
+               crop_cam2img=np.asarray(ref['cam2img'], np.float64),
+               crop_img_shape=np.asarray(ref['img_shape']))
+    np.savez_compressed(os.path.join(HERE, 'pipeline_meta.npz'), **out)
+    print('pipeline_meta', {k: v.shape for k, v in out.items()})
+
+
+def reference_checks(ns):
+    from oracle.ref_loader import REFERENCE_ROOT
+    state_dict_layout_case(ns)
+    config_blocks_case(REFERENCE_ROOT)
+    voxel_sample_case(ns)
+    bev_stage_small_case(ns)
+    spp_lastconv_case(ns)
+    pipeline_meta_case(REFERENCE_ROOT)
+
+
 def main():
+    from tests.util import FIXTURE_THREADS
     ns = load_reference()
     torch.manual_seed(0)
+    torch.set_num_threads(FIXTURE_THREADS)
     if 'frustum' in sys.argv[1:]:
         frustum_case(ns)
         return
@@ -174,12 +309,16 @@ def main():
     if 'neck_mt' in sys.argv[1:]:
         neck_multitile_case(ns)
         return
+    if 'checks' in sys.argv[1:]:
+        reference_checks(ns)
+        return
     for name, spec in KITTI_CASES.items():
         kitti_case(ns, name, spec)
     neck_case(ns)
     neck_multitile_case(ns)
     frustum_case(ns)
     bev_stage_case(ns)
+    reference_checks(ns)
 
 
 if __name__ == '__main__':

@@ -1,6 +1,7 @@
 """CPU tests of the host-side mirror: registry/config plumbing, state_dict
 contract, geometry packing, C-ABI library symbols."""
 import ctypes
+import json
 import os
 import re
 import shutil
@@ -13,9 +14,9 @@ import torch
 import depth_from_motion_b200 as pkg
 from depth_from_motion_b200 import capi, modules, registry
 from depth_from_motion_b200 import synthetic as syn
+from tests.util import DFM_CONFIGS, GOLDEN, STATE_DICT_MODULES
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = '/root/reference'
 
 
 def test_registry_builds_by_type():
@@ -71,32 +72,27 @@ def test_state_dict_contract():
         'voxel_convs.0.0.gn.weight': (32,), 'voxel_convs.0.0.gn.bias': (32,)}
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree not mounted')
 def test_state_dict_matches_reference_modules():
-    from oracle.ref_loader import load_reference
-    ns = load_reference()
-    cfg = syn.depth_cfg_for(16)
-    a = modules.DfMBackbone(in_channels=32, depth_cfg=cfg).state_dict()
-    b = ns.DfMBackbone(in_channels=32, depth_cfg=cfg).state_dict()
-    assert list(a) == list(b)
-    assert all(a[k].shape == b[k].shape for k in a)
-    for ours, ref in ((modules.DfMNeck(64, 256, num_frames=2), ns.DfMNeck(64, 256, num_frames=2)),
-                      (modules.OutdoorImVoxelNeck(64, 256), ns.OutdoorImVoxelNeck(64, 256)),
-                      (modules.FrustumToVoxel(), ns.FrustumToVoxel()),
-                      (modules.FrustumToVoxel(num_3dconvs=2, cat_img_feature=False),
-                       ns.FrustumToVoxel(num_3dconvs=2, cat_img_feature=False))):
-        a, b = ours.state_dict(), ref.state_dict()
-        assert list(a) == list(b) and all(a[k].shape == b[k].shape for k in a)
+    """Key order and shapes equal those of the reference modules' state_dicts
+    (tests/golden/state_dict_layout.json)."""
+    with open(os.path.join(GOLDEN, 'state_dict_layout.json')) as f:
+        gold = json.load(f)
+    assert sorted(gold) == sorted(STATE_DICT_MODULES)
+    for name, make in STATE_DICT_MODULES.items():
+        sd = make(modules).state_dict()
+        assert [[k, list(v.shape)] for k, v in sd.items()] == gold[name], name
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree not mounted')
-@pytest.mark.parametrize('cfg_name', [
-    'dfm_r34_1x8_kitti-3d-3class.py',
-    'multiview-dfm_r101_dcn_2x16_waymoD5-3d-3class_camsync.py',
-    'multiview-dfm_r101_dcn_2x16_waymoD5-3d-3class_camsync_10sweeps.py'])
-def test_reference_configs_parse_and_build_hot_path(cfg_name):
-    """configs/dfm/*.py load unchanged: parse -> build the hot-path modules by type."""
-    cfg = registry.Config.fromfile(os.path.join(REF, 'configs/dfm', cfg_name))
+@pytest.mark.parametrize('cfg_name', DFM_CONFIGS)
+def test_reference_configs_parse_and_build_hot_path(cfg_name, tmp_path):
+    """The hot-path blocks of configs/dfm/*.py, as the reference parses them
+    (tests/golden/config_model_blocks.json), load from a flat config file and build the
+    hot-path modules by type."""
+    with open(os.path.join(GOLDEN, 'config_model_blocks.json')) as f:
+        blocks = json.load(f)[cfg_name]
+    path = tmp_path / cfg_name
+    path.write_text(f'model = {blocks!r}\n')
+    cfg = registry.Config.fromfile(str(path))
     model = cfg.model
     if model['type'] == 'DfM':
         bs = dict(model['backbone_stereo'])

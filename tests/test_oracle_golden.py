@@ -9,7 +9,18 @@ import torch
 
 from depth_from_motion_b200 import synthetic as syn
 from oracle import dfm_oracle as O
-from tests.util import GOLDEN, KITTI_CASES, load_kitti_case
+from tests.util import FIXTURE_THREADS, GOLDEN, KITTI_CASES, load_kitti_case
+
+
+@pytest.fixture(autouse=True)
+def _fixture_threads():
+    """The CPU kernels split their reductions (float64 sums, convolutions) by the number of
+    intra-op threads, so the oracle reproduces the fixtures to the bit only with the thread
+    count they were generated with, whatever the host's core count."""
+    saved = torch.get_num_threads()
+    torch.set_num_threads(FIXTURE_THREADS)
+    yield
+    torch.set_num_threads(saved)
 
 
 def test_points_img2cam_kat():
@@ -165,28 +176,14 @@ def test_frustum_to_voxel_matches_reference_fixture():
                                                      (288, 304, 20)))
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/mmdet3d'), reason='reference tree not mounted')
 @pytest.mark.parametrize('flip,aligned', [(False, True), (True, True), (False, False)])
 def test_voxel_sample_matches_reference_source(flip, aligned):
     """SURVEY.md row a8 (oracle only): the restatement against the reference function executed
-    verbatim (point_fusion.py:324-410)."""
-    import torch.nn.functional as F
-    from oracle.ref_loader import load_reference, reference_function
-    ns = load_reference()
-    ref = reference_function('mmdet3d/models/fusion_layers/point_fusion.py', 'voxel_sample',
-                             dict(torch=torch, F=F, points_img2cam=ns.points_img2cam))
-    g = torch.Generator().manual_seed(3)
-    vox = torch.randn(1, 6, 20, 16, 8, generator=g)
-    vrange, vsize = [0.0, -8.0, -2.0, 20.0, 8.0, 2.0], [1.0, 1.0, 0.5]
-    depths = torch.linspace(2.0, 18.0, 16)
-    # lidar -> image: camera looks along +x
-    k = torch.tensor([[40., 0, 32, 0], [0, 40., 16, 0], [0, 0, 1, 0], [0, 0, 0, 1]])
-    l2c = torch.tensor([[0., -1, 0, 0], [0, 0, -1, 0.3], [1, 0, 0, 0.1], [0, 0, 0, 1]])
-    proj = k @ l2c
-    args = (vox, vrange, vsize, depths, proj, 4, torch.tensor([1.02, 0.98]),
-            torch.tensor([1.0, 2.0]), flip, (32, 64), (30, 62))
-    a = ref(*args, aligned=aligned)
-    b = O.voxel_sample(*args, aligned=aligned)
+    verbatim (point_fusion.py:324-410), stored in tests/golden/voxel_sample.npz."""
+    from tests.util import voxel_sample_args
+    gold = np.load(os.path.join(GOLDEN, 'voxel_sample.npz'))
+    a = torch.from_numpy(gold[f'flip{int(flip)}_aligned{int(aligned)}'])
+    b = O.voxel_sample(*voxel_sample_args(flip), aligned=aligned)
     assert a.shape == b.shape == (1, 6, 4, 8, 16)
     assert torch.equal(a, b)
     assert float(a.abs().sum()) > 0
@@ -210,42 +207,31 @@ def test_bev_stage_matches_reference_fixture():
     assert outs[0].shape[1] == 18 and outs[1].shape[1] == 42 and outs[2].shape[1] == 12
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/mmdet3d'), reason='reference tree not mounted')
 def test_bev_stage_oracle_equals_reference_source():
-    """Bit-for-bit against the reference classes executed in place (only where mounted)."""
-    from oracle.ref_loader import load_reference
-    ns = load_reference()
-    c = syn.make_bev_case(seed=5, nz=5, ny=12, nx=16)
-    gn = dict(type='GN', num_groups=32, requires_grad=True)
-    bev = ns.BEVHourglass(160, 64, norm_cfg=gn).eval()
-    head = ns.LIGAAnchor3DHead(3, 64, 64, 6, norm_cfg=gn).eval()
-    bev.load_state_dict(c['bev'], strict=True)
-    head.load_state_dict(c['head'], strict=True)
-    x = c['volume'].reshape(1, 160, 12, 16)
+    """Bit-for-bit against the reference classes executed verbatim on a 12 x 16 BEV grid
+    (tests/golden/bev_stage_small.npz)."""
+    from tests.util import BEV_SMALL_CASE
+    gold = np.load(os.path.join(GOLDEN, 'bev_stage_small.npz'))
+    c = syn.make_bev_case(**BEV_SMALL_CASE)
     with torch.no_grad():
-        _, feat = bev(x)
-        ref = head.forward_single(feat)
         got = O.dfm_bev_stage(c['bev'], c['head'], c['volume'])
-    for a, b in zip(got, ref):
-        assert torch.equal(a, b)
+    for a, key in zip(got, ('cls_score', 'bbox_pred', 'dir_cls_preds')):
+        assert torch.equal(a, torch.from_numpy(gold[key])), key
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/mmdet3d'), reason='reference tree not mounted')
 def test_spp_unet_lastconv_equals_reference_module():
     """SURVEY.md section 8(f) row 2: the oracle restatement of SPPUNetNeck.lastconv against the
-    reference class executed in place (spp_unet_neck.py:60-75, :110)."""
-    from oracle.ref_loader import load_reference
-    ns = load_reference()
-    gn = dict(type='GN', num_groups=32, requires_grad=True)
-    m = ns.SPPUNetNeck(in_channels=[3, 64, 128, 128, 128], start_level=2, sem_channels=[128, 32],
-                       stereo_channels=[32, 32], with_upconv=True, cat_img_feature=True,
-                       norm_cfg=gn).eval()
-    p = {k: v for k, v in m.state_dict().items() if k.startswith('lastconv')}
+    reference class executed verbatim (spp_unet_neck.py:60-75, :110): its parameters and output
+    are stored in tests/golden/spp_unet_lastconv.npz."""
+    from tests.util import spp_lastconv_input
+    gold = dict(np.load(os.path.join(GOLDEN, 'spp_unet_lastconv.npz')))
+    y = torch.from_numpy(gold.pop('y'))
+    p = {k: torch.from_numpy(v) for k, v in gold.items()}
     assert sorted(p) == ['lastconv.0.conv.weight', 'lastconv.0.gn.bias', 'lastconv.0.gn.weight',
                          'lastconv.1.weight']
-    x = torch.randn(1, 32, 24, 40, generator=torch.Generator().manual_seed(4))
+    x = spp_lastconv_input()
     with torch.no_grad():
-        assert torch.equal(m.lastconv(x), O.spp_unet_lastconv(p, x))
+        assert torch.equal(y, O.spp_unet_lastconv(p, x))
     # the mirror takes the same keys
     from depth_from_motion_b200 import modules
     modules.SPPUNetNeckTail().load_state_dict(p, strict=True)

@@ -1,18 +1,12 @@
 """CPU tests of the input-side metadata (SURVEY.md section 8(f) row 4) against the reference's
 own VideoPipeline / RandomCrop3D code executed verbatim on the demo KITTI sample."""
-import copy
 import os
-import pickle
 
 import numpy as np
-import pytest
 
 from depth_from_motion_b200 import pipeline_meta as pm
 from depth_from_motion_b200 import synthetic as syn
-
-REF = '/root/reference'
-needs_ref = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'mmdet3d')),
-                               reason='reference tree not mounted')
+from tests.util import GOLDEN
 
 
 def test_cur2prevs_matches_recorded_demo_geometry():
@@ -40,29 +34,17 @@ def test_quaternion_matrix():
     assert np.allclose(m[:3, :3] @ m[:3, :3].T, np.eye(3))
 
 
-@needs_ref
 def test_video_meta_matches_reference_pipeline():
-    from oracle.ref_loader import reference_class
-    info = pickle.load(open(os.path.join(REF, 'demo/data/kitti/kitti_000008_infos.pkl'), 'rb'))[0]
-    img_info = dict(filename='x.png', cam2global=info['image']['cam2global'],
-                    sweeps=[dict(data_path=s['data_path'], cam2global=s['cam2global'])
-                            for s in info['image']['sweeps']])
-
-    class Compose:   # the image transforms are out of scope: identity
-        def __init__(self, t):
-            pass
-
-        def __call__(self, r):
-            r['img'] = 0
-            return r
-
-    VP = reference_class('mmdet3d/datasets/pipelines/loading.py', 'VideoPipeline',
-                         dict(np=np, copy=copy, Compose=Compose))
+    """Against the reference VideoPipeline executed verbatim on the geometry of its demo KITTI
+    sample (both stored in tests/golden/pipeline_meta.npz)."""
+    gold = np.load(os.path.join(GOLDEN, 'pipeline_meta.npz'))
+    img_info = dict(filename='x.png', cam2global=gold['cam2global'],
+                    sweeps=[dict(data_path=str(p), cam2global=m)
+                            for p, m in zip(gold['sweep_paths'], gold['sweep_cam2global'])])
     for nref, rand in ((1, False), (3, False), (2, True)):
-        np.random.seed(7)
-        ref = VP([], num_ref_imgs=nref, random=rand)(dict(img_info=copy.deepcopy(img_info)))
+        ref = gold[f'cur2prevs_n{nref}_random{int(rand)}']
         got = pm.video_meta(img_info, nref, rand, rng=np.random.RandomState(7))
-        assert np.array_equal(ref['cur2prevs'], got['cur2prevs'])
+        assert np.array_equal(ref, got['cur2prevs'])
         assert [m for m in got['ref_filenames']] == \
             [img_info['sweeps'][i]['data_path'] for i in got['ref_ids']]
     # the three sweeps are what synthetic.KITTI_CUR2PREV records (nearest first)
@@ -70,27 +52,16 @@ def test_video_meta_matches_reference_pipeline():
     assert np.allclose(allp, syn.KITTI_CUR2PREV, atol=1e-6)
 
 
-@needs_ref
 def test_crop3d_meta_matches_reference():
-    from oracle.ref_loader import reference_class
-
-    class RandomCrop:   # mmdet base: only what _crop_data touches
-        def __init__(self, **kw):
-            self.bbox_clip_border = kw.get('bbox_clip_border', True)
-            self.bbox2label, self.bbox2mask = {}, {}
-
-    RC = reference_class('mmdet3d/datasets/pipelines/transforms_3d.py', 'RandomCrop3D',
-                         dict(np=np, RandomCrop=RandomCrop))
-    rc = RC(crop_size=(320, 1280), rel_offset_h=(0.3, 1.0))
-    img = np.zeros((375, 1242, 3), dtype=np.uint8)
-    np.random.seed(3)
-    ref = rc._crop_data(dict(img=img, cam2img=syn.KITTI_P2.copy()), (320, 1280), True)
+    """Against RandomCrop3D._crop_data executed verbatim (crop (320, 1280) of a 375 x 1242
+    image, np.random.seed(3); stored in tests/golden/pipeline_meta.npz)."""
+    gold = np.load(os.path.join(GOLDEN, 'pipeline_meta.npz'))
     rng = np.random.RandomState(3)
-    x1, y1 = pm.random_crop_offsets(img.shape, (320, 1280), (0.3, 1.0), (0., 1.), rng)
+    x1, y1 = pm.random_crop_offsets((375, 1242, 3), (320, 1280), (0.3, 1.0), (0., 1.), rng)
     cam, off = pm.crop3d_meta(syn.KITTI_P2, x1, y1)
-    assert off == ref['crop_offset']
-    assert np.allclose(cam, ref['cam2img'], atol=1e-9)
-    assert ref['img_shape'][:2] == (320, 1242)
+    assert off == gold['crop_offset'].tolist()
+    assert np.allclose(cam, gold['crop_cam2img'], atol=1e-9)
+    assert tuple(gold['crop_img_shape'][:2].tolist()) == (320, 1242)
 
 
 def test_backbone_img_meta_feeds_geometry_packing():

@@ -7,6 +7,8 @@ import torch
 from depth_from_motion_b200 import synthetic as syn
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
+# intra-op CPU threads tests/golden/make_golden.py computes the fixtures with
+FIXTURE_THREADS = 8
 
 # must match tests/golden/make_golden.py
 KITTI_CASES = {
@@ -72,3 +74,49 @@ def load_frustum_case():
     for k in ('stereo', 'cost', 'sem'):
         c[k] = torch.from_numpy(gold[k])
     return c, gold
+
+
+# must match tests/golden/make_golden.py: the modules whose state_dict layout (key order and
+# shapes) is stored in state_dict_layout.json; `ns` is either the package's `modules` or the
+# reference namespace, both have these class names
+STATE_DICT_MODULES = {
+    'DfMBackbone': lambda ns: ns.DfMBackbone(in_channels=32, depth_cfg=syn.depth_cfg_for(16)),
+    'DfMNeck': lambda ns: ns.DfMNeck(64, 256, num_frames=2),
+    'OutdoorImVoxelNeck': lambda ns: ns.OutdoorImVoxelNeck(64, 256),
+    'FrustumToVoxel': lambda ns: ns.FrustumToVoxel(),
+    'FrustumToVoxel(num_3dconvs=2, cat_img_feature=False)':
+        lambda ns: ns.FrustumToVoxel(num_3dconvs=2, cat_img_feature=False),
+}
+
+# the shipped configs/dfm/*.py and, per detector type, the blocks of their `model` dict that
+# the hot path is built from (stored in config_model_blocks.json)
+DFM_CONFIGS = ('dfm_r34_1x8_kitti-3d-3class.py',
+               'multiview-dfm_r101_dcn_2x16_waymoD5-3d-3class_camsync.py',
+               'multiview-dfm_r101_dcn_2x16_waymoD5-3d-3class_camsync_10sweeps.py')
+CONFIG_MODEL_BLOCKS = {
+    'DfM': ('type', 'depth_cfg', 'voxel_cfg', 'backbone_stereo', 'depth_head',
+            'feature_transformation', 'backbone_3d', 'bbox_head_3d'),
+    'MultiViewDfM': ('type', 'neck_3d'),
+}
+
+
+def voxel_sample_args(flip):
+    """Inputs of the voxel_sample fixture (voxel_sample.npz): a camera looking along +x."""
+    g = torch.Generator().manual_seed(3)
+    vox = torch.randn(1, 6, 20, 16, 8, generator=g)
+    vrange, vsize = [0.0, -8.0, -2.0, 20.0, 8.0, 2.0], [1.0, 1.0, 0.5]
+    depths = torch.linspace(2.0, 18.0, 16)
+    # lidar -> image: camera looks along +x
+    k = torch.tensor([[40., 0, 32, 0], [0, 40., 16, 0], [0, 0, 1, 0], [0, 0, 0, 1]])
+    l2c = torch.tensor([[0., -1, 0, 0], [0, 0, -1, 0.3], [1, 0, 0, 0.1], [0, 0, 0, 1]])
+    proj = k @ l2c
+    return (vox, vrange, vsize, depths, proj, 4, torch.tensor([1.02, 0.98]),
+            torch.tensor([1.0, 2.0]), flip, (32, 64), (30, 62))
+
+
+# must match tests/golden/make_golden.py
+BEV_SMALL_CASE = dict(seed=5, nz=5, ny=12, nx=16)
+
+
+def spp_lastconv_input():
+    return torch.randn(1, 32, 24, 40, generator=torch.Generator().manual_seed(4))
